@@ -6,7 +6,7 @@ Primary line (one JSON object on stdout, rank 0): PatchMatch Mpixels/s on config
 GPU (weak scaling, no data-path collective in photometric mode).  The BA metric (LM iterations/s on
 B3) rides along under the "ba" key when the BA path is built.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
   python -m torch.distributed.run --nproc-per-node N ... bench.py --gpus N ...
 
 value  : device-resident (inputs already in HBM), CUDA-event time of b200pm_run, max over ranks.
@@ -171,8 +171,42 @@ def _oracle_ba_sample(noisy, max_iters=100):
     return steps / dt, dt, f"B3 problem (500 cams, 300k pts, 2M obs), full solve ({steps} LM iterations, limit {max_iters}), ITERATIVE_SCHUR, oracle port"
 
 
-def bench_ba(steps, warmup, peak, peak_src, with_cpu):
-    """BA leg: LM iterations/s on config B3 (500 SIMPLE_RADIAL cameras, 300k points, 2M observations, Schur-PCG)."""
+DUMP_LIMIT = 64 << 20      # bytes that --dump-outputs may write in all
+DUMP_SAMPLE = 1 << 17      # rows kept of an output too large to store whole
+
+
+def _fixed_sample(n, k=DUMP_SAMPLE):
+    """Sorted indices of a seeded sample of k of range(n) (all of them when n <= k): the same rows in every run."""
+    import numpy as np
+    if n <= k:
+        return np.arange(n)
+    return np.sort(np.random.default_rng(0).choice(n, k, replace=False))
+
+
+def _ba_outputs(prefix, flat, summary, sample_points=False):
+    """What a caller of solve_flat receives: the refined blocks of `flat` and the summary's costs."""
+    import numpy as np
+    pts = flat.points[_fixed_sample(len(flat.points))] if sample_points else flat.points
+    return {f"{prefix}_poses": flat.poses, f"{prefix}_cam_params": flat.cam_params, f"{prefix}_points": pts,
+            f"{prefix}_cost": np.array([summary.initial_cost, summary.final_cost], np.float64)}
+
+
+def dump_outputs(directory, outputs):
+    """Writes every array of `outputs` as DIR/<name>.npy in float32 / float64 (integer and mask arrays as float32)."""
+    import numpy as np
+    arrays = {k: np.ascontiguousarray(v if v.dtype in (np.float32, np.float64) else v.astype(np.float32))
+              for k, v in outputs.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT:
+        raise SystemExit(f"--dump-outputs: {total} bytes exceed the {DUMP_LIMIT}-byte limit")
+    os.makedirs(directory, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(directory, k + ".npy"), a)
+
+
+def bench_ba(steps, warmup, peak, peak_src, with_cpu, outputs=None):
+    """BA leg: LM iterations/s on config B3 (500 SIMPLE_RADIAL cameras, 300k points, 2M observations, Schur-PCG).
+    `outputs`, when given, receives the solution of the last timed solve."""
     from colmap_b200.bundle_adjustment import ITERATIVE_SCHUR, BundleAdjustmentOptions, solve_flat
     noisy = _b3_problem()
     o = BundleAdjustmentOptions(linear_solver_type=ITERATIVE_SCHUR)
@@ -201,6 +235,8 @@ def bench_ba(steps, warmup, peak, peak_src, with_cpu):
            "roofline": {"bound": "hbm", "kernel": "ba_schur_spmv_warp_smem_kernel + ba_cam_stream_loop_kernel (one implicit-Schur product)", "achieved": achieved, "peak": peak, "unit": "GB/s",
                         "frac": achieved / peak, "traffic": _ncu_traffic("ba_schur_spmv_kernel"), "peak_source": peak_src,
                         "algorithmic_bytes_per_launch": alg, "launch_ms": spmv_launch_ms}}
+    if outputs is not None:
+        outputs.update(_ba_outputs("ba_b3", f, s))
     if with_cpu:
         v, dt, sample = _oracle_ba_sample(noisy)
         out["cpu_baseline"] = {"value": v, "unit": "LM iterations/s", "cores": os.cpu_count(), "kind": "port",
@@ -264,8 +300,9 @@ def bench_c4(rank, world, local_rank, images_total):
             "quality": {"valid_frac": valid, "median_rel_depth_err": float(np.median(rel)) if rel else None}}
 
 
-def bench_b5(steps, warmup, rank, world, local_rank, comm):
-    """BA leg on config B5 (2000 cameras, 2M points, 12M observations, mixed models), points sharded over the ranks."""
+def bench_b5(steps, warmup, rank, world, local_rank, comm, outputs=None):
+    """BA leg on config B5 (2000 cameras, 2M points, 12M observations, mixed models), points sharded over the ranks.
+    `outputs`, when given, receives the solution of the last timed solve (a fixed sample of the points)."""
     import numpy as np
     import torch
     import torch.distributed as dist
@@ -297,6 +334,8 @@ def bench_b5(steps, warmup, rank, world, local_rank, comm):
             dev_ms += s.solve_ms
     if world > 1:
         dev_ms = max_over_ranks(dev_ms, "cuda"); wall_ms = max_over_ranks(wall_ms, "cuda")
+    elif outputs is not None:
+        outputs.update(_ba_outputs("ba_b5", local, s, sample_points=True))
     return {"metric": "ba_lm_iterations_per_s", "value": lm / (dev_ms * 1e-3), "unit": "LM iterations/s", "dtype": "f64",
             "n_gpus": world, "scaling": "strong", "ms_per_step": dev_ms / steps, "lm_iterations_per_solve": lm / steps,
             "config": {"workload": B5_WORKLOAD},
@@ -334,7 +373,7 @@ def bench_ba_sharded(steps, warmup, rank, world, local_rank, with_b5=False):
     b5 = None
     if with_b5:
         try:
-            b5 = bench_b5(min(steps, 2), 1, rank, world, local_rank, comm)
+            b5 = bench_b5(steps, 1, rank, world, local_rank, comm)
         except Exception as e:
             b5 = {"error": repr(e)}
     collective = ("one-shot all-reduce kernel over NVLink peer memory (cudaIpc symmetric buffers), one launch per collective"
@@ -489,7 +528,14 @@ def main():
                     help="images of the C4-shaped workspace leg: -1 = 3 per GPU when 8 GPUs run (the configuration's GPU count), "
                          "else skipped; 0 = skip; 200 = the full configuration")
     ap.add_argument("--b5", type=int, default=1, help="BA config B5 leg (2000 cameras, 2M points, 12M observations; strong scaling over the ranks): 1 = run, 0 = skip")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step of each single-GPU leg returned (rank 0) as DIR/<name>.npy, so that "
+                         "two builds can be compared output for output; the inputs are seeded")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
 
     rank = _env_int("RANK", 0)
     world = _env_int("WORLD_SIZE", 1)
@@ -559,6 +605,12 @@ def main():
     valid = depth > 0
     rel = np.abs(depth - sc["depth_gt"])[valid] / sc["depth_gt"][valid]
     quality = dict(valid_frac=float(valid.mean()), median_rel_depth_err=float(np.median(rel)))
+    outputs = {} if args.dump_outputs and rank == 0 else None
+    if outputs is not None:
+        # the per-source maps (N x H x W) are kept at a fixed sample of pixels
+        px = _fixed_sample(W * H)
+        outputs.update(pm_depth=depth, pm_normal=pm.GetNormalMap(), pm_sel_prob=pm.GetSelProbMap().reshape(N, -1)[:, px],
+                       pm_consistency_mask=pm.GetConsistencyMask().reshape(N, -1)[:, px])
     pm.close()
 
     # ---------------- end-to-end leg through the public API with host buffers
@@ -635,18 +687,20 @@ def main():
                                     "sample": sample, "seconds": dt}
         if not args.no_ba and world == 1:
             try:
-                line["ba"] = bench_ba(args.steps, args.warmup, peak, peak_src, not args.no_cpu_baseline)
+                line["ba"] = bench_ba(args.steps, args.warmup, peak, peak_src, not args.no_cpu_baseline, outputs)
             except Exception as e:  # the primary metric must still be reported
                 line["ba"] = {"error": repr(e)}
         if ba_sharded is not None:
             line["ba"] = ba_sharded
         if want_b5 and not distributed and not args.no_ba:
             try:
-                line.setdefault("ba", {})["b5"] = bench_b5(min(args.steps, 2), 1, rank, world, local_rank, None)
+                line.setdefault("ba", {})["b5"] = bench_b5(args.steps, 1, rank, world, local_rank, None, outputs)
             except Exception as e:
                 line.setdefault("ba", {})["b5"] = {"error": repr(e)}
         if c4 is not None:
             line["c4"] = c4
+        if outputs is not None:
+            dump_outputs(args.dump_outputs, outputs)
         print(json.dumps(line), flush=True)
     if distributed:
         dist.destroy_process_group()

@@ -1,6 +1,8 @@
 """GPU parity tier for the bundle-adjustment path: b200ba_solve (CUDA, fp64) against the CPU oracle on the same
 inputs.  Bar (BASELINE.json north_star): final cost / residual and parameters within 1e-5 relative; residual
 counts exact; constant blocks bit-identical."""
+import os
+
 import numpy as np
 import pytest
 
@@ -235,28 +237,20 @@ def test_assemble_then_solve_on_the_gpu():
 
 
 def test_cross_backend_with_the_reference_caspar_solver():
-    """The reference's own GPU backend (generated Caspar solver, fp32, compiled in place into oracle/_ref) on the same
-    problem - the cross-backend check of bundle_adjustment_caspar_test.cc:957-1022 (MergedCalibMatchesCeres: one shared
-    SIMPLE_RADIAL camera, principal point refined; focal within 20, principal point within 10, extra within 1.5e-2 in
-    fp32) with our solver in the role of Ceres, plus the final cost.  Caspar fixes one frame only (scale left free), so
-    costs and intrinsics are compared, poses are not."""
-    import ref_caspar
-    if not ref_caspar.available():
-        pytest.skip("oracle/_ref/libcaspar_ref.so not built (needs /root/reference at build time)")
-    gt, noisy = synthesize_ba_problem(12, 2000, 8, models=(SIMPLE_RADIAL,), shared_camera=True, seed=13,
-                                      point2D_stddev=0.5, point3D_stddev=0.1, translation_stddev=0.05, rotation_stddev_deg=0.3)
-    _gauge(noisy)
-    o = BundleAdjustmentOptions(refine_principal_point=True)
-    a, b = noisy.copy(), noisy.copy()
-    for f in (a, b):
-        f.pose_constant, f.pose_fixed_dim = noisy.pose_constant, noisy.pose_fixed_dim
+    """The reference's own GPU backend (generated Caspar solver, fp32) on the same problem, as stored in
+    tests/golden/ba_reference_caspar.npz (tests/golden/make_golden.py --reference) - the cross-backend check of
+    bundle_adjustment_caspar_test.cc:957-1022 (MergedCalibMatchesCeres: one shared SIMPLE_RADIAL camera, principal point
+    refined; focal within 20, principal point within 10, extra within 1.5e-2 in fp32) with our solver in the role of
+    Ceres, plus the final cost.  Caspar fixes one frame only (scale left free), so costs and intrinsics are compared,
+    poses are not."""
+    import make_golden
+    a, o = make_golden.caspar_case()
     sg = solve_flat(o, a)
-    rc = ref_caspar.solve(b, o)
-    # (caspar::SolveResult::initial_score is never written by the generated solver, solver.cc:2408-2410)
-    msg = f"ours {sg.final_cost} ({a.cam_params}) caspar {rc} ({b.cam_params})"
-    assert rc["num_residuals"] == sg.num_residuals, msg
-    assert abs(rc["final_cost"] - sg.final_cost) <= 2e-2 * sg.final_cost, msg
-    pa, pb = a.cam_params.reshape(-1, 4), b.cam_params.reshape(-1, 4)
+    rc = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "ba_reference_caspar.npz"))
+    msg = f"ours {sg.final_cost} ({a.cam_params}) caspar {float(rc['final_cost'])} ({rc['cam_params']})"
+    assert int(rc["num_residuals"]) == sg.num_residuals, msg
+    assert abs(float(rc["final_cost"]) - sg.final_cost) <= 2e-2 * sg.final_cost, msg
+    pa, pb = a.cam_params.reshape(-1, 4), rc["cam_params"].reshape(-1, 4)
     assert np.abs(pa[:, 0] - pb[:, 0]).max() < 20.0 and np.abs(pa[:, 1:3] - pb[:, 1:3]).max() < 10.0, msg
     assert np.abs(pa[:, 3] - pb[:, 3]).max() < 1.5e-2, msg
 

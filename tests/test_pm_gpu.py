@@ -177,31 +177,33 @@ def test_full_hd_properties():
     assert np.isfinite(got["sel_prob"]).all() and (got["sel_prob"] >= 0).all() and (got["sel_prob"] <= 1).all()
 
 
-def test_statistical_parity_with_the_real_reference_cuda():
-    """oracle/_ref/libpm_ref.so is COLMAP's own patch_match_cuda.cu (unmodified, built against stub headers, PTX JIT).
-    It is stochastic and numerically different (fast-math, texture filtering), so the comparison is statistical:
-    same completeness and accuracy against the analytic ground truth, and per-pixel agreement of the two depth maps."""
-    import ref_pm
-    if not ref_pm.available():
-        pytest.skip("oracle/_ref/libpm_ref.so not built (needs /root/reference at build time)")
-    sc = make_patch_match_scene(480, 270, 8, seed=0)
-    o = PatchMatchOptions(depth_min=sc["depth_min"], depth_max=sc["depth_max"], geom_consistency=False, gpu_index="0")
-    ref = ref_pm.run(o, sc["problem"])
+def _reference_parity(w, h):
+    """Runs the CUDA path on the scene of make_golden.reference_parity_case and loads what COLMAP's own
+    patch_match_cuda.cu (unmodified, built against stub headers, PTX JIT) produced for it: whole-map statistics of its
+    depth against the ground truth, and its depth / normal maps on a regular pixel grid.  Returns (stored fixture,
+    whole-map statistics of our depth, our depth and normal on the same grid)."""
+    import make_golden
+    sc, o = make_golden.reference_parity_case(w, h)
+    z = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", make_golden.reference_parity_name(w, h)))
     got = _run_cuda(o, sc["problem"])
-    gt = sc["depth_gt"]
+    s = int(z["step"])
+    return z, make_golden.depth_stats(got["depth"], sc["depth_gt"]), got["depth"][::s, ::s], got["normal"][:, ::s, ::s]
 
-    def stats(d):
-        v = d > 0
-        rel = np.abs(d - gt)[v] / gt[v]
-        return v.mean(), np.median(rel), (rel < 1e-3).mean()
-    (va, ma, fa), (vb, mb, fb) = stats(ref["depth"]), stats(got["depth"])
+
+def test_statistical_parity_with_the_real_reference_cuda():
+    """tests/golden/pm_reference_cuda_480x270_grid.npz: the reference PatchMatchCuda on a 480x270 scene.  It is
+    stochastic and numerically different (fast-math, texture filtering), so the comparison is statistical: same
+    completeness and accuracy against the analytic ground truth over the whole map, and per-pixel agreement of the two
+    depth maps on the stored grid (3600 pixels)."""
+    ref, (vb, mb, fb), depth, normal = _reference_parity(480, 270)
+    va, ma, fa = float(ref["valid_frac"]), float(ref["median_rel_err"]), float(ref["frac_rel_err_lt_1e_3"])
     assert abs(va - vb) < 0.01 and abs(fa - fb) < 0.02 and mb < 2 * ma + 1e-5
-    both = (ref["depth"] > 0) & (got["depth"] > 0)
-    dd = np.abs(ref["depth"] - got["depth"])[both]
+    both = (ref["depth"] > 0) & (depth > 0)
+    dd = np.abs(ref["depth"] - depth)[both]
     assert both.mean() > 0.97
     assert (dd < 1e-3).mean() > 0.8          # depth ~ 5 m: 1e-3 m = 2e-4 relative
     assert (dd < 1e-4).mean() > 0.25         # north_star: within 1e-4 m where both converge
-    nn = (ref["normal"] * got["normal"]).sum(0)[both]
+    nn = (ref["normal"] * normal).sum(0)[both]
     assert np.median(nn) > 0.999
 
 
@@ -261,27 +263,19 @@ def test_c2_full_size_bit_exact_vs_oracle():
 
 
 def test_c2_full_size_statistical_parity_with_the_real_reference_cuda():
-    """C2 (all 5 iterations) against COLMAP's own PatchMatchCuda on the same GPU.  STATISTICAL parity (the reference is
-    stochastic in its float details: fast-math, 9-bit texture weights): the figures of
-    profiles/pm_ref_compare_1920x1080.json (61 % of pixels within 1e-4 m, 98.7 % within 1e-3 m, 5 m scene) pinned with
-    a margin."""
-    import ref_pm
-    if not ref_pm.available():
-        pytest.skip("oracle/_ref/libpm_ref.so not built (needs /root/reference at build time)")
-    sc = make_patch_match_scene(1920, 1080, 8, seed=0)
-    o = PatchMatchOptions(depth_min=sc["depth_min"], depth_max=sc["depth_max"], geom_consistency=False, gpu_index="0")
-    ref = ref_pm.run(o, sc["problem"])
-    got = _run_cuda(o, sc["problem"])
-    gt = sc["depth_gt"]
-    va, vb = ref["depth"] > 0, got["depth"] > 0
-    assert abs(va.mean() - vb.mean()) < 0.005 and vb.mean() > 0.99
-    ea = np.median(np.abs(ref["depth"] - gt)[va] / gt[va]); eb = np.median(np.abs(got["depth"] - gt)[vb] / gt[vb])
+    """C2 (all 5 iterations) against COLMAP's own PatchMatchCuda (tests/golden/pm_reference_cuda_1920x1080_grid.npz).
+    STATISTICAL parity (the reference is stochastic in its float details: fast-math, 9-bit texture weights): the figures
+    of profiles/pm_ref_compare_1920x1080.json (61 % of pixels within 1e-4 m, 98.7 % within 1e-3 m, 5 m scene) pinned
+    with a margin; whole-map completeness and accuracy, per-pixel agreement on the stored grid (8160 pixels)."""
+    ref, (vb, eb, _), depth, normal = _reference_parity(1920, 1080)
+    va, ea = float(ref["valid_frac"]), float(ref["median_rel_err"])
+    assert abs(va - vb) < 0.005 and vb > 0.99
     assert eb < 1.5 * ea + 1e-6 and eb < 5e-5
-    both = va & vb
-    dd = np.abs(ref["depth"] - got["depth"])[both]
+    both = (ref["depth"] > 0) & (depth > 0)
+    dd = np.abs(ref["depth"] - depth)[both]
     assert (dd < 1e-4).mean() > 0.55          # north_star: within 1e-4 m where both converge
     assert (dd < 1e-3).mean() > 0.97
-    assert np.median((ref["normal"] * got["normal"]).sum(0)[both]) > 0.9999
+    assert np.median((ref["normal"] * normal).sum(0)[both]) > 0.9999
 
 
 def test_two_phase_with_device_resident_maps_equals_the_host_round_trip():

@@ -330,11 +330,11 @@ def test_run_workspace_fails_loudly_without_a_workspace_or_a_gpu(tmp_path):
     (ws / "sparse" / "cameras.bin").write_bytes(np.array([1], np.uint64).tobytes() + b"\x01\x00")          # count 1, then truncated
     with pytest.raises(WorkspaceError, match="truncated"):
         run_workspace(o, str(ws))
-    # a structurally valid (tiny) workspace: without a device the call must refuse, not fall back
-    import torch
-    if torch.cuda.is_available():
-        pytest.skip("needs a box without a GPU")
+    # a structurally valid (tiny) workspace: without a device the call must refuse, not fall back.  The call runs in a
+    # child process that sees no CUDA device, so that this holds on a machine with a GPU as well.
+    import re
     import struct
+    import subprocess
     cam = struct.pack("<Q", 1) + struct.pack("<IiQQ", 1, 1, 64, 48) + struct.pack("<4d", 50.0, 50.0, 32.0, 24.0)
     (ws / "sparse" / "cameras.bin").write_bytes(cam)
     imgs = struct.pack("<Q", 2)
@@ -350,6 +350,16 @@ def test_run_workspace_fails_loudly_without_a_workspace_or_a_gpu(tmp_path):
     (ws / "images").mkdir()
     for i in (1, 2):
         (ws / "images" / f"im{i}.pgm").write_bytes(b"P5\n64 48\n255\n" + bytes(64 * 48))
-    with pytest.raises(WorkspaceError, match="CUDA|device|GPU"):
-        run_workspace(o, str(ws), gpu_indices=[0])
+    child = ("import sys\n"
+             "from colmap_b200.mvs_workspace import WorkspaceError, run_workspace\n"
+             "from colmap_b200.patch_match import PatchMatchOptions\n"
+             "try:\n"
+             "    run_workspace(PatchMatchOptions(), sys.argv[1], gpu_indices=[0])\n"
+             "except WorkspaceError as e:\n"
+             "    print(e)\n"
+             "    sys.exit(3)\n")
+    r = subprocess.run([sys.executable, "-c", child, str(ws)], capture_output=True, text=True, timeout=300, cwd=ROOT,
+                       env=dict(os.environ, CUDA_VISIBLE_DEVICES=""))
+    assert r.returncode == 3, r.stdout + r.stderr
+    assert re.search("CUDA|device|GPU", r.stdout), r.stdout
     assert not (ws / "stereo" / "depth_maps").exists() or not any((ws / "stereo" / "depth_maps").iterdir())
